@@ -171,6 +171,38 @@ def synth_hash(stream, index):
     return z ^ (z >> 31)
 
 
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, groups, keys, nq):
+    """Writes what the timed paths returned in their last step as float32 / float64 .npy files, so that two builds can be
+    compared output for output: the GROUP BY rows (the 128-bit SUM(v) rounded to float64), and each query's top-k decoded
+    from its sortable keys in hit order (score desc, doc asc; doc -1 marks an empty slot). If the top-k arrays would not
+    fit in DUMP_BYTES, a fixed seeded sample of the queries is written, with their indices in bm25_query."""
+    import serenedb_b200 as sdb
+    out = {}
+    if groups is not None:
+        out["groupby_key"] = groups["key"].astype(np.float64)
+        out["groupby_count"] = groups["count"].astype(np.float64)
+        out["groupby_sum_v"] = np.array([float(s) for s in sdb.sum_i128(groups)], np.float64)
+        out["groupby_sum_w"] = groups["sum_f64"].astype(np.float64)
+        out["groupby_count_w"] = groups["cnt_f64"].astype(np.float64)
+    if keys is not None:
+        k = keys.view(np.uint64).reshape(nq, -1)
+        room = DUMP_BYTES - sum(a.nbytes for a in out.values()) - (1 << 16)   # headroom for the .npy headers
+        take = min(nq, room // (k.shape[1] * 12 + 8))
+        q = np.arange(nq) if take == nq else np.sort(np.random.default_rng(0).choice(nq, take, replace=False))
+        k = np.sort(k[q], axis=1)[:, ::-1]
+        doc = (~k & np.uint64(0xFFFFFFFF)).astype(np.float64)
+        doc[k == 0] = -1
+        out["bm25_query"] = q.astype(np.float64)
+        out["bm25_score"] = (k >> np.uint64(32)).astype(np.uint32).view(np.float32)
+        out["bm25_doc"] = doc
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
+
+
 def make_queries(nq, n_terms=N_TERMS, stream=7):
     """Two-term disjunctions, pairs drawn from the synthetic terms (SURVEY §8d); query 0 is the named
     case p = (0.10, 0.01) => terms 5 and 59."""
@@ -304,7 +336,9 @@ def main():
     quiet_stdout()
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10,
+                    help="timed steps of the headline GROUP BY and BM25 legs and of their e2e legs; the secondary probes "
+                         "(BM25 pruning-off roofline, HBM-resident index, zonemap, configs[0], configs[3]) keep fixed counts")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--rows", type=int, default=100_000_000, help="table rows per GPU")
@@ -317,7 +351,11 @@ def main():
     ap.add_argument("--cpu-rows", type=int, default=100_000_000)
     ap.add_argument("--cpu-queries", type=int, default=256)
     ap.add_argument("--cpu-threads", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step as DIR/<name>.npy (float32/float64, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -329,6 +367,8 @@ def main():
             args.rows = 125_000_000
         if args.docs == 10_000_000:
             args.docs = 12_500_000
+    if args.dump_outputs and (args.impl != "ours" or world > 1):
+        ap.error("--dump-outputs needs --impl ours on one GPU")
     if args.impl == "reference":
         args.cpu_rows = min(args.cpu_rows, args.rows)
         run_reference(args, rank)
@@ -478,7 +518,7 @@ def main():
                 torch.cuda.synchronize()
             return escan.groupby_finalize(key_min, span, d_i64.data_ptr(), d_f64.data_ptr(), span)
 
-        e_steps = max(1, min(args.steps, 5))
+        e_steps = args.steps
         e_raw_ms = None
         for use_packed in (False, True):
             eres = e2e_step(use_packed)
@@ -549,6 +589,7 @@ def main():
         line["cpu_baseline"] = cpu_gb
 
     oseg = odc = osdl = None
+    bm25_keys, nq = None, 0
     # ------------------------------------------------------------------ BM25 (configs[2])
     if not args.skip_bm25:
         n_docs = args.docs
@@ -604,6 +645,9 @@ def main():
         barrier()
         # headline: shipped configuration (block-max pruning on: lead mode for pairs whose long list can be probed)
         bm_ms, tk_ms, mg_ms, bm_launches, clocks2 = timed_bm25(bm25_step, args.steps, "default")
+        if args.dump_outputs:
+            ctx.sync()
+            bm25_keys = keys.cpu().numpy()     # the last timed step's top-k keys, before later legs overwrite them
         hits_p, n_p, tot_pruned = [x.copy() for x in batch.run_host()] if dist is None else (None, None, None)   # run_host reuses its buffers
         # roofline leg: the same batch with pruning off -- every list of every query is decoded, so the touched bytes
         # are exactly the lists' encoded bytes (what the numerator claims)
@@ -619,7 +663,7 @@ def main():
         batch.run_host()
         barrier()
         ctx.timer_start()
-        e_steps2 = max(1, min(args.steps, 5))
+        e_steps2 = args.steps
         for _ in range(e_steps2):
             if dist is None:
                 hits, n_out, total_e = batch.run_host()
@@ -803,6 +847,8 @@ def main():
                                                 "sample": "%d concurrent copies of the query" % ncpu4}}
         seg4.close()
         line["other_configs"] = other
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, res, bm25_keys, nq)
     if rank == 0:
         emit_line(line)
     if dist is not None:

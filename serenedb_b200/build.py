@@ -1,8 +1,10 @@
 """Builds libsdbg.so (the sm_100a kernels + C ABI) in-tree with nvcc. No JIT cache: the .so lives
 under serenedb_b200/_lib/ so it travels to the GPU box with the repo snapshot."""
+import atexit
 import os
 import shutil
 import subprocess
+import tempfile
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
@@ -39,16 +41,25 @@ def build(force=False, verbose=False):
         if os.path.exists(LIB_PATH):
             return LIB_PATH  # GPU box without sources changed: use the shipped build
         raise RuntimeError("nvcc not found and no prebuilt libsdbg.so")
-    os.makedirs(LIB_DIR, exist_ok=True)
-    tmp = LIB_PATH + ".tmp"
+    lib_path = LIB_PATH
+    if os.access(LIB_DIR if os.path.isdir(LIB_DIR) else HERE, os.W_OK):
+        os.makedirs(LIB_DIR, exist_ok=True)
+    else:
+        # read-only tree, e.g. when the import finds the sources newer than the library: the rebuilt library goes to a
+        # private temporary directory, never into the tree. The build step itself (build_adapters, the oracle) still
+        # writes the tree.
+        tmp_dir = tempfile.mkdtemp(prefix="sdbg-")
+        atexit.register(shutil.rmtree, tmp_dir, True)
+        lib_path = os.path.join(tmp_dir, "libsdbg.so")
+    tmp = lib_path + ".tmp"
     cmd = [nvcc] + NVCC_FLAGS + (["-Xptxas", "-v"] if verbose else []) + ["-o", tmp] + SOURCES + ["-lpthread"]
     res = subprocess.run(cmd, capture_output=True, text=True)
     if res.returncode != 0:
         raise RuntimeError("nvcc failed:\n" + res.stdout + res.stderr)
-    os.replace(tmp, LIB_PATH)
+    os.replace(tmp, lib_path)
     if verbose:
         print(res.stderr)
-    return LIB_PATH
+    return lib_path
 
 
 HOST_DIR = os.path.join(HERE, "host")

@@ -2,9 +2,12 @@
 
 TEST INFRASTRUCTURE. Only tests/, __graft_entry__.smoke() and bench.py's CPU legs import this.
 """
+import atexit
 import ctypes as C
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -12,16 +15,33 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 ORACLE_DIR = os.path.join(ROOT, "oracle")
 LIB_PATH = os.path.join(ORACLE_DIR, "_build", "liboracle.so")
 REF_SIMDCOMP = os.path.join(ORACLE_DIR, "_ref", "libsimdcomp_ref.so")
+_tmp_lib = None   # a library built outside a read-only tree, reused for the rest of the process
 
 
 def build(force=False):
+    """Compiles the oracle when its sources are newer than the library; returns the library's path."""
+    global _tmp_lib
+    if _tmp_lib is not None and not force:
+        return _tmp_lib
     src = [os.path.join(ORACLE_DIR, f) for f in ("oracle.cpp", "oracle.h", "Makefile")]
     stale = (not os.path.exists(LIB_PATH)) or any(
         os.path.getmtime(s) > os.path.getmtime(LIB_PATH) for s in src)
+    path = LIB_PATH
     if force or stale:
-        subprocess.check_call(["make", "-C", ORACLE_DIR, "-s"], stdout=subprocess.DEVNULL)
+        make = ["make", "-C", ORACLE_DIR, "-s"]
+        out_dir = os.path.dirname(LIB_PATH)
+        if not os.access(out_dir if os.path.isdir(out_dir) else ORACLE_DIR, os.W_OK):
+            # read-only tree: build into a private temporary directory, never into the tree
+            out_dir = tempfile.mkdtemp(prefix="oracle-")
+            atexit.register(shutil.rmtree, out_dir, True)
+            make.append("BUILD=" + out_dir)
+            path = os.path.join(out_dir, "liboracle.so")
+        subprocess.check_call(make, stdout=subprocess.DEVNULL)
+        if path != LIB_PATH:
+            _tmp_lib = path
     if os.path.isdir("/root/reference/third_party/simdcomp/src") and not os.path.exists(REF_SIMDCOMP):
         subprocess.check_call(["make", "-C", ORACLE_DIR, "-s", "ref"], stdout=subprocess.DEVNULL)
+    return path
 
 
 class BM25Stats(C.Structure):
@@ -64,8 +84,7 @@ def lib():
     global _lib
     if _lib is not None:
         return _lib
-    build()
-    L = C.CDLL(LIB_PATH)
+    L = C.CDLL(build())
     u32p, u8p, u64p, f32p = (C.POINTER(C.c_uint32), C.POINTER(C.c_uint8), C.POINTER(C.c_uint64),
                              C.POINTER(C.c_float))
     vp = C.c_void_p

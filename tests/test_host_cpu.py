@@ -143,22 +143,6 @@ def test_cpp_adapters_build_and_fail_loudly_without_gpu():
     assert res.returncode == 3 and '"error": -2' in res.stdout
 
 
-def test_mock_headers_match_the_reference():
-    """Every `//@ref file:lines` block of host/irs_mock.hpp repeats the cited reference declarations token for token, so the
-    adapters override the real virtual surface (FillBlock, GetMutable, FetchScoreArgs, ScoreCollector(Tag) included).
-    Needs the reference tree: skipped on boxes without it."""
-    import importlib.util
-    import os
-    import pytest
-    if not os.path.isdir("/root/reference/libs/iresearch"):
-        pytest.skip("no reference tree on this box")
-    spec = importlib.util.spec_from_file_location("check_mock", os.path.join(os.path.dirname(__file__), "..", "tools", "check_mock.py"))
-    m = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(m)
-    blocks, decls, problems = m.check("/root/reference")
-    assert blocks >= 6 and decls >= 60 and not problems, problems
-
-
 def _for_decode(headers, words, rows):
     """Independent (pure Python) decoder of the bit-packed column format described in include/sdbg.h."""
     out = np.zeros(rows, np.int64)

@@ -1,69 +1,10 @@
-"""Oracle codec vs the reference: bit packing against the reference's own simdcomp (oracle/_ref),
-block encoder choice + round trips (format_block_128.hpp), StreamVByte round trips."""
-import ctypes as C
-import os
-
+"""Oracle codec: block encoder choice + round trips (format_block_128.hpp), StreamVByte round trips."""
 import numpy as np
 import pytest
 
 import orc
 
 RNG = np.random.default_rng(0x5EDB2026)
-
-
-def _ref():
-    if not os.path.exists(orc.REF_SIMDCOMP):
-        orc.build()
-    if not os.path.exists(orc.REF_SIMDCOMP):
-        pytest.skip("oracle/_ref/libsimdcomp_ref.so not built (no /root/reference here)")
-    L = C.CDLL(orc.REF_SIMDCOMP)
-    L.simdpackwithoutmask.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32]
-    L.simdunpack.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32]
-    L.simdpackwithoutmaskd1.argtypes = [C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint32]
-    L.simdunpackd1.argtypes = [C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint32]
-    return L
-
-
-@pytest.mark.parametrize("bits", list(range(1, 32)))
-def test_pack_matches_reference_simdcomp(bits):
-    """The restated bit layout equals third_party/simdcomp byte for byte (both directions)."""
-    R = _ref()
-    L = orc.lib()
-    for _ in range(4):
-        vals = RNG.integers(0, 1 << bits, size=128, dtype=np.uint64).astype(np.uint32)
-        mine = np.zeros(4 * bits, np.uint32)
-        theirs = np.zeros(4 * bits, np.uint32)
-        L.orc_pack128(orc.ptr(vals), orc.ptr(mine), bits)
-        R.simdpackwithoutmask(orc.ptr(vals), orc.ptr(theirs), bits)
-        assert np.array_equal(mine, theirs)
-        back = np.zeros(128, np.uint32)
-        L.orc_unpack128(orc.ptr(theirs), orc.ptr(back), bits)
-        assert np.array_equal(back, vals)
-        back2 = np.zeros(128, np.uint32)
-        R.simdunpack(orc.ptr(mine), orc.ptr(back2), bits)
-        assert np.array_equal(back2, vals)
-
-
-@pytest.mark.parametrize("bits", list(range(2, 32)))
-def test_pack_d1_matches_reference_simdcomp(bits):
-    R = _ref()
-    L = orc.lib()
-    for _ in range(4):
-        hi = min((1 << bits) - 1, (0xFFFFFFFF // 130))
-        deltas = RNG.integers(1, hi + 1, size=128, dtype=np.uint64)
-        prev = int(RNG.integers(0, 1000))
-        vals = (prev + np.cumsum(deltas)).astype(np.uint32)
-        mine = np.zeros(4 * bits, np.uint32)
-        theirs = np.zeros(4 * bits, np.uint32)
-        L.orc_pack128_d1(prev, orc.ptr(vals), orc.ptr(mine), bits)
-        R.simdpackwithoutmaskd1(prev, orc.ptr(vals), orc.ptr(theirs), bits)
-        assert np.array_equal(mine, theirs)
-        back = np.zeros(128, np.uint32)
-        L.orc_unpack128_d1(prev, orc.ptr(theirs), orc.ptr(back), bits)
-        assert np.array_equal(back, vals)
-        back2 = np.zeros(128, np.uint32)
-        R.simdunpackd1(prev, orc.ptr(mine), orc.ptr(back2), bits)
-        assert np.array_equal(back2, vals)
 
 
 def _sorted_docs(n, prev, mean_gap):
@@ -159,21 +100,3 @@ def test_streamvbyte_layout_and_roundtrip():
         back = np.zeros(length, np.uint32)
         assert L.orc_svb_delta_decode(orc.ptr(buf), orc.ptr(back), length, 9) == n
         assert np.array_equal(back, d)
-
-
-def test_block_decode_through_reference_simdcomp():
-    """Same bytes decode identically with the scalar restatement and the reference's SSE unpack."""
-    if not orc.use_simdcomp_ref(True):
-        pytest.skip("no oracle/_ref")
-    try:
-        for gap in (3.0, 40.0, 9000.0):
-            d = _sorted_docs(128, 100, gap)
-            buf = orc.encode_doc_block(d, 100)
-            back, _ = orc.decode_doc_block(buf, 128, 100)
-            assert np.array_equal(back, d)
-            f = RNG.integers(1, 40, size=128).astype(np.uint32)
-            fb = orc.encode_freq_block(f)
-            back, _ = orc.decode_freq_block(fb, 128)
-            assert np.array_equal(back, f)
-    finally:
-        orc.use_simdcomp_ref(False)
